@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N --steps K --warmup W
     python bench.py --workload cfg2|cfg3|cfg4|cfg3n ...       (default cfg3 = the configuration the metric is quoted on)
     python bench.py --global-batch 4096 ...                   (strong scaling: BASELINE config 3's batch split over N GPUs)
+    python bench.py --dump-outputs DIR ...                    (what the last timed step decoded, as DIR/*.npy)
 
 Workloads (config.workload; tools/bench_inputs.py): the synthetic source images S(w,h,seed) of SURVEY.md 8d encoded by the
 REFERENCE ENCODER (oracle/_ref/jpeg, named in config.encoder; the repo's own generator only where that binary is absent),
@@ -257,6 +258,31 @@ def bind_to_gpu_numa_node(index):
     return "none"
 
 
+# fixed sample of the decoded frames for --dump-outputs: one 4K frame alone is 25 MB of samples
+DUMP_SEED, DUMP_FRAMES, DUMP_SAMPLES_PER_FRAME = 2024, 8, 1 << 20
+
+
+def dump_outputs(dec, out, directory):
+    """Writes what one decode of the batch delivered to its caller, as arrays two builds can be compared on:
+    frame_status.npy   float64 [frames]               status of every frame (0 = decoded)
+    frame_sums.npy     float64 [frames, components]   sum of every sample of each component of every frame
+    frame_samples.npy  float32 [8, 2^20]              the samples at fixed seeded positions of 8 fixed seeded frames
+    sample_frames.npy  float64 [8]                    which frames those are"""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    views = [dec.frame_view(out, i) for i in range(dec.n)]
+    np.save(os.path.join(directory, "frame_status.npy"), np.array([dec.status(i) for i in range(dec.n)], dtype=np.float64))
+    sums = torch.stack([v.reshape(-1, v.shape[-1]).sum(0, dtype=torch.float64) for v in views])
+    np.save(os.path.join(directory, "frame_sums.npy"), sums.cpu().numpy())
+    rng = np.random.default_rng(DUMP_SEED)
+    picked = np.sort(rng.choice(dec.n, size=min(DUMP_FRAMES, dec.n), replace=False))
+    n = min([DUMP_SAMPLES_PER_FRAME] + [views[i].numel() for i in picked])
+    samples = [views[i].reshape(-1)[torch.from_numpy(rng.integers(0, views[i].numel(), size=n)).to(out.device)] for i in picked]
+    np.save(os.path.join(directory, "frame_samples.npy"), torch.stack(samples).float().cpu().numpy())
+    np.save(os.path.join(directory, "sample_frames.npy"), picked.astype(np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -274,7 +300,13 @@ def main():
     ap.add_argument("--p2d-chunks", type=int, default=2, help="pinned_to_device_rgb: chunks per step (each: H2D + index + kernels on its own stream)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one decoded as DIR/*.npy (rank 0's frames)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -381,6 +413,8 @@ def main():
     barrier()
     clocks = sampler.stop()
     total_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(dec, out, args.dump_outputs)
     t = torch.tensor([total_ms], device="cuda")
     if dist is not None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -391,7 +425,7 @@ def main():
 
     # the once-per-upload restart index, timed alone (idempotent re-run)
     idx_ms = []
-    for _ in range(3):
+    for _ in range(args.steps):
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record(stream)
         dec.reindex(stream)
@@ -408,7 +442,7 @@ def main():
     # stream around each stage
     ent_ms, rec_ms, uns_ms = [], [], []
     dec.enable_timing(True)
-    for _ in range(3):
+    for _ in range(args.steps):
         dec.decode(out, stream)
         torch.cuda.synchronize()
         a, b = dec.last_timing()
@@ -479,7 +513,7 @@ def main():
         for _ in range(2):
             p2d_step()
         barrier()
-        psteps = max(2, min(args.steps, 5))
+        psteps = args.steps
         t0 = time.perf_counter()
         for _ in range(psteps):
             p2d_step()
@@ -574,7 +608,7 @@ def main():
         barrier()
         counters["h2d"] = counters["d2h"] = 0
         t0 = time.perf_counter()
-        esteps = max(2, min(args.steps, 5))
+        esteps = args.steps
         for i in range(esteps):
             last_bd = e2e_step(keep_last=(i == esteps - 1))
         barrier()

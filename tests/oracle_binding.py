@@ -121,7 +121,7 @@ class Oracle:
 
 
 def build():
-    """Compiles the C restatement (always) and, where /root/reference exists, the reference itself."""
+    """Compiles the C restatement (always) and, where the reference sources exist, the reference itself."""
     subprocess.run(["make", "-s", "-C", ORACLE_DIR, "all"], check=True)
 
 
@@ -129,10 +129,6 @@ def load():
     if not os.path.exists(LIB):
         build()
     return Oracle(ctypes.CDLL(LIB))
-
-
-def have_reference():
-    return os.path.exists(REF_HARNESS) and os.path.exists(REF_CLI)
 
 
 def reference_decode(jpg_path, tmp_raw):

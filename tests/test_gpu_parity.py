@@ -394,7 +394,7 @@ def test_reference_cli_linked_against_the_b200_library(built, golden_pixels, tmp
     import subprocess
     exe = os.path.join(ROOT, "oracle", "_ref", "jpeg_b200")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/jpeg_b200 is built where /root/reference exists (oracle/Makefile)")
+        pytest.skip("oracle/_ref/jpeg_b200 is built where the reference build exists (oracle/Makefile)")
     for name in NAMES:
         out = str(tmp_path / (name + ".pnm"))
         r = subprocess.run([exe, os.path.join(GOLDEN, name + ".jpg"), out], capture_output=True, text=True)
@@ -599,7 +599,7 @@ def test_reference_cli_writes_12bit_frames_through_the_b200_library(built, tmp_p
     import subprocess
     exe = os.path.join(ROOT, "oracle", "_ref", "jpeg_b200")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/jpeg_b200 is built where /root/reference exists (oracle/Makefile)")
+        pytest.skip("oracle/_ref/jpeg_b200 is built where the reference build exists (oracle/Makefile)")
     wants = np.load(os.path.join(DEEP12, "deep12_pixels.npz"))
     for name in D12NAMES:
         out = str(tmp_path / (name + ".pnm"))
@@ -639,7 +639,7 @@ def test_reference_cli_without_upsampling_through_the_b200_library(built, tmp_pa
     import subprocess
     exe = os.path.join(ROOT, "oracle", "_ref", "jpeg_b200")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/jpeg_b200 is built where /root/reference exists (oracle/Makefile)")
+        pytest.skip("oracle/_ref/jpeg_b200 is built where the reference build exists (oracle/Makefile)")
     fx, names = _plane_fixtures()
     for name in names:
         out = str(tmp_path / "o")
@@ -697,7 +697,7 @@ def test_reference_cli_decodes_xt_through_the_b200_library(built, tmp_path):
     import subprocess
     exe = os.path.join(ROOT, "oracle", "_ref", "jpeg_b200")
     if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/jpeg_b200 is built where /root/reference exists (oracle/Makefile)")
+        pytest.skip("oracle/_ref/jpeg_b200 is built where the reference build exists (oracle/Makefile)")
     fx = np.load(os.path.join(XT, "xt_pixels.npz"))
     for name in [n for n in XTNAMES if not n.endswith("__nimpl")]:
         out = str(tmp_path / (name + ".pnm"))

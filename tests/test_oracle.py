@@ -1,8 +1,11 @@
-"""CPU: pins the oracle (oracle/jpeg_oracle.c) -- against the committed golden vectors that the unmodified
-reference produced (tests/golden/make_golden.py) and, where the reference build is present, against the
-reference itself on fresh streams."""
+"""CPU: pins the oracle (oracle/jpeg_oracle.c) against what the unmodified reference made of the same streams -- the
+golden vectors (tests/golden/make_golden.py ...) and the streams built below, whose reference decodes are stored as shape
+and SHA-256 of the pixels in tests/golden/reference_decodes.json (tests/golden/make_reference_decodes.py)."""
 import glob
+import hashlib
+import json
 import os
+import re
 
 import numpy as np
 import pytest
@@ -16,6 +19,63 @@ NAMES = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN, 
 @pytest.fixture(scope="module")
 def golden_pixels():
     return np.load(os.path.join(GOLDEN, "golden_pixels.npz"))
+
+
+REFERENCE_DECODES = os.path.join(GOLDEN, "reference_decodes.json")
+REFERENCE_ENCODED = os.path.join(GOLDEN, "reference_encoded")
+
+
+def reference_key(kind, params):
+    """Name of a case in reference_decodes.json: (72, 40, (2, 2), 3, 60) -> '<kind>__72_40_2_2_3_60'."""
+    return kind + "__" + "_".join(re.findall(r"[0-9A-Za-z]+", str(params)))
+
+
+def pixel_digest(px):
+    return {"shape": list(px.shape), "sha256": hashlib.sha256(np.ascontiguousarray(px).tobytes()).hexdigest()}
+
+
+def reference_decode(kind, params):
+    """Shape and SHA-256 of the reference's pixels for a case, None where the reference refused the stream."""
+    ref = json.load(open(REFERENCE_DECODES))[reference_key(kind, params)]
+    return None if ref == "refused" else ref
+
+
+def same_pixels(px, ref):
+    return px.dtype == np.uint8 and pixel_digest(px) == ref
+
+
+def synthetic_stream(w, h, sub, z, q):
+    from libjpeg_b200 import synth
+    return synth.encode(synth.source_image(w, h, 7 * w + h), q, sub, z).tobytes()
+
+
+def hot_stream(w, h, sub, z, dcq):
+    from libjpeg_b200 import synth
+    return oracle_binding.with_dc_quantiser(synth.encode(synth.source_image(w, h, 5), 75, sub, z), dcq)
+
+
+def damaged_stream(damage):
+    from libjpeg_b200 import synth
+    return oracle_binding.with_restart_damage(synth.encode(synth.source_image(200, 136, 3), 75, (2, 2), 2), damage)
+
+
+def variant_stream(flags, w, h, sub, z):
+    from libjpeg_b200 import synth
+    return synth.encode(synth.source_image(w, h, 5), 80, sub, z, flags).tobytes()
+
+
+def four_component_stream(w, h, sub, z):
+    from libjpeg_b200 import synth
+    return oracle_binding.with_fourth_component(synth.encode(synth.source_image(w, h, 5), 80, sub, z, 1))
+
+
+SYNTHETIC = [(72, 40, (2, 2), 3, 60), (31, 47, (2, 2), 0, 85), (64, 32, (1, 1), 8, 92), (90, 33, (2, 1), 2, 70), (45, 90, (1, 2), 6, 70)]
+HOT = [(96, 80, (2, 2), 3, 255), (200, 120, (2, 1), 0, 160), (64, 64, (1, 1), 4, 255), (130, 70, (1, 2), 2, 200)]
+# sampling factors the reference encoder's -s takes; the streams it wrote are stored beside its decodes
+OTHER_SUBSAMPLING = ["1x1,4x1,4x1", "1x1,3x2,3x2", "1x1,2x3,2x3", "1x1,1x4,1x4", "1x1,3x4,3x4", "1x1,4x3,4x3", "1x1,2x1,4x2"]
+VARIANTS = [(1, 70, 50, (2, 2), 5), (1, 64, 48, (1, 1), 0), (2, 40, 40, (2, 2), 3), (6, 40, 40, (2, 1), 0), (7, 33, 47, (1, 2), 4)]
+FOUR_COMPONENT = [(64, 48, (1, 1), 4), (70, 50, (2, 2), 5), (100, 37, (2, 1), 0), (33, 90, (1, 2), 3)]
+NO_COLOR_TRANSFORM = ["c420_96x80_z6_q75", "c444_64x64_z16_q90", "c422_100x60_z5_q80"]
 
 
 @pytest.mark.parametrize("name", NAMES)
@@ -32,34 +92,23 @@ def test_golden_covers_all_vectors(golden_pixels):
     assert sorted(golden_pixels.files) == NAMES and len(NAMES) >= 12
 
 
-@pytest.mark.skipif(not oracle_binding.have_reference(), reason="reference build (oracle/_ref) not present")
-@pytest.mark.parametrize("w,h,sub,z,q", [(72, 40, (2, 2), 3, 60), (31, 47, (2, 2), 0, 85), (64, 32, (1, 1), 8, 92),
-                                          (90, 33, (2, 1), 2, 70), (45, 90, (1, 2), 6, 70)])
-def test_oracle_matches_reference_on_synthetic_streams(oracle, built, tmp_path, w, h, sub, z, q):
+@pytest.mark.parametrize("w,h,sub,z,q", SYNTHETIC)
+def test_oracle_matches_reference_on_synthetic_streams(oracle, built, w, h, sub, z, q):
     """Streams from the repo's own generator, decoded by the real reference and by the oracle."""
-    from libjpeg_b200 import synth
-    data = synth.encode(synth.source_image(w, h, 7 * w + h), q, sub, z)
-    jpg = tmp_path / "s.jpg"
-    jpg.write_bytes(data.tobytes())
-    ref = oracle_binding.reference_decode(str(jpg), str(tmp_path / "s.raw"))
+    ref = reference_decode("synthetic", (w, h, sub, z, q))
     assert ref is not None
-    rc, px = oracle.decode(data.tobytes())
-    assert rc == 0 and np.array_equal(px, ref)
+    rc, px = oracle.decode(synthetic_stream(w, h, sub, z, q))
+    assert rc == 0 and same_pixels(px, ref)
 
 
-@pytest.mark.skipif(not oracle_binding.have_reference(), reason="reference build (oracle/_ref) not present")
-@pytest.mark.parametrize("w,h,sub,z,dcq", [(96, 80, (2, 2), 3, 255), (200, 120, (2, 1), 0, 160), (64, 64, (1, 1), 4, 255), (130, 70, (1, 2), 2, 200)])
-def test_oracle_matches_reference_beyond_the_usual_sample_range(oracle, built, tmp_path, w, h, sub, z, dcq):
+@pytest.mark.parametrize("w,h,sub,z,dcq", HOT)
+def test_oracle_matches_reference_beyond_the_usual_sample_range(oracle, built, w, h, sub, z, dcq):
     """DC quantiser patched to a large value: IDCT samples leave int16 and the 32-bit colour range (the reference
     computes the colour matrix in 64 bits); the oracle must follow the reference there too."""
-    from libjpeg_b200 import synth
-    data = oracle_binding.with_dc_quantiser(synth.encode(synth.source_image(w, h, 5), 75, sub, z), dcq)
-    jpg = tmp_path / "hot.jpg"
-    jpg.write_bytes(data)
-    ref = oracle_binding.reference_decode(str(jpg), str(tmp_path / "hot.raw"))
+    ref = reference_decode("hot", (w, h, sub, z, dcq))
     assert ref is not None
-    rc, px = oracle.decode(data)
-    assert rc == 0 and np.array_equal(px, ref)
+    rc, px = oracle.decode(hot_stream(w, h, sub, z, dcq))
+    assert rc == 0 and same_pixels(px, ref)
 
 
 def test_oracle_idct_dc_only(oracle):
@@ -112,22 +161,13 @@ def test_oracle_matches_3x_4x_subsampling_golden(oracle, name):
     assert np.array_equal(px.reshape(want.shape), want)
 
 
-@pytest.mark.skipif(not oracle_binding.have_reference(), reason="reference build (oracle/_ref) not present")
-@pytest.mark.parametrize("sub", ["1x1,4x1,4x1", "1x1,3x2,3x2", "1x1,2x3,2x3", "1x1,1x4,1x4", "1x1,3x4,3x4", "1x1,4x3,4x3", "1x1,2x1,4x2"])
-def test_oracle_matches_reference_on_other_subsampling(oracle, tmp_path, sub):
-    """Fresh streams from the reference's encoder (its CLI takes the sampling factors), decoded by reference and oracle."""
-    import subprocess
-    from libjpeg_b200 import synth
-    w, h = 75, 61
-    ppm = tmp_path / "in.ppm"
-    ppm.write_bytes(b"P6\n%d %d\n255\n" % (w, h) + synth.source_image(w, h, 17).tobytes())
-    jpg = tmp_path / "s.jpg"
-    r = subprocess.run([oracle_binding.REF_CLI, "-q", "80", "-bl", "-s", sub, "-z", "3", str(ppm), str(jpg)],
-                       capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr
-    ref = oracle_binding.reference_decode(str(jpg), str(tmp_path / "s.raw"))
-    rc, px = oracle.decode(jpg.read_bytes())
-    assert rc == 0 and np.array_equal(px.reshape(ref.shape), ref)
+@pytest.mark.parametrize("sub", OTHER_SUBSAMPLING)
+def test_oracle_matches_reference_on_other_subsampling(oracle, sub):
+    """Streams of the reference's encoder (its CLI takes the sampling factors: `jpeg -q 80 -bl -s <sub> -z 3` on S(75, 61, 17)),
+    decoded by reference and oracle."""
+    ref = reference_decode("subsampling", sub)
+    rc, px = oracle.decode(open(os.path.join(REFERENCE_ENCODED, reference_key("subsampling", sub) + ".jpg"), "rb").read())
+    assert rc == 0 and same_pixels(px, ref)
 
 
 DAMAGED = os.path.join(GOLDEN, "damaged")
@@ -144,20 +184,15 @@ def test_oracle_matches_damaged_golden(oracle, name):
     assert np.array_equal(px.reshape(want.shape), want)
 
 
-@pytest.mark.skipif(not oracle_binding.have_reference(), reason="reference build (oracle/_ref) not present")
 @pytest.mark.parametrize("damage", oracle_binding.RESTART_DAMAGES)
-def test_oracle_resynchronises_like_the_reference(oracle, tmp_path, damage):
+def test_oracle_resynchronises_like_the_reference(oracle, built, damage):
     """Restart markers out of sequence, missing, duplicated, buried in garbage: same verdict and same pixels as the reference."""
-    from libjpeg_b200 import synth
-    b = oracle_binding.with_restart_damage(synth.encode(synth.source_image(200, 136, 3), 75, (2, 2), 2), damage)
-    jpg = tmp_path / "d.jpg"
-    jpg.write_bytes(bytes(b))
-    ref = oracle_binding.reference_decode(str(jpg), str(tmp_path / "d.raw"))
-    rc, px = oracle.decode(bytes(b))
+    ref = reference_decode("damage", damage)
+    rc, px = oracle.decode(damaged_stream(damage))
     if ref is None:
         assert rc != 0
     else:
-        assert rc == 0 and np.array_equal(px.reshape(ref.shape), ref)
+        assert rc == 0 and same_pixels(px, ref)
 
 
 DEEP12 = os.path.join(GOLDEN, "deep12")
@@ -187,19 +222,13 @@ def test_progressive_golden_is_complete():
     assert set(np.load(os.path.join(PROGRESSIVE, "progressive_pixels.npz")).files) == set(PNAMES)
 
 
-@pytest.mark.skipif(not oracle_binding.have_reference(), reason="reference build (oracle/_ref) not present")
-@pytest.mark.parametrize("flags,w,h,sub,z", [(1, 70, 50, (2, 2), 5), (1, 64, 48, (1, 1), 0), (2, 40, 40, (2, 2), 3), (6, 40, 40, (2, 1), 0),
-                                            (7, 33, 47, (1, 2), 4)])
-def test_oracle_matches_reference_on_stream_variants(oracle, built, tmp_path, flags, w, h, sub, z):
+@pytest.mark.parametrize("flags,w,h,sub,z", VARIANTS)
+def test_oracle_matches_reference_on_stream_variants(oracle, built, flags, w, h, sub, z):
     """One scan per component (flag 1), SOF1 header (2), 16-bit DQT (4): accepted by the reference, same pixels."""
-    from libjpeg_b200 import synth
-    data = synth.encode(synth.source_image(w, h, 5), 80, sub, z, flags)
-    jpg = tmp_path / "v.jpg"
-    jpg.write_bytes(data.tobytes())
-    ref = oracle_binding.reference_decode(str(jpg), str(tmp_path / "v.raw"))
+    ref = reference_decode("variant", (flags, w, h, sub, z))
     assert ref is not None
-    rc, px = oracle.decode(data.tobytes())
-    assert rc == 0 and np.array_equal(px, ref)
+    rc, px = oracle.decode(variant_stream(flags, w, h, sub, z))
+    assert rc == 0 and same_pixels(px, ref)
 
 
 NOEOI = os.path.join(GOLDEN, "noeoi")
@@ -227,16 +256,12 @@ def test_noeoi_fixtures_cover_both_verdicts():
     assert sorted(status) == NENAMES and 0 in status.values() and -1025 in status.values()
 
 
-@pytest.mark.skipif(not oracle_binding.have_reference(), reason="reference build (oracle/_ref) not present")
-def test_zrl_that_steps_over_position_63_ends_the_block_silently(oracle, tmp_path):
+def test_zrl_that_steps_over_position_63_ends_the_block_silently(oracle):
     """sequentialscan.cpp:717-719: after a ZRL the reference re-tests k <= 63 and leaves the block without an error."""
-    data = oracle_binding.zrl_overrun_stream()
-    jpg = tmp_path / "z.jpg"
-    jpg.write_bytes(data)
-    ref = oracle_binding.reference_decode(str(jpg), str(tmp_path / "z.raw"))
+    ref = reference_decode("zrl", ())
     assert ref is not None
-    rc, px = oracle.decode(data)
-    assert rc == 0 and np.array_equal(px.reshape(ref.shape), ref)
+    rc, px = oracle.decode(oracle_binding.zrl_overrun_stream())
+    assert rc == 0 and same_pixels(px, ref)
 
 
 DNL = os.path.join(GOLDEN, "dnl")
@@ -254,34 +279,20 @@ def test_oracle_reads_the_height_from_the_dnl_marker(oracle, name):
     assert np.array_equal(got[:-1], px[name + "__ref_dnl"][:-1])
 
 
-@pytest.mark.skipif(not oracle_binding.have_reference(), reason="reference build (oracle/_ref) not present")
-@pytest.mark.parametrize("w,h,sub,z", [(64, 48, (1, 1), 4), (70, 50, (2, 2), 5), (100, 37, (2, 1), 0), (33, 90, (1, 2), 3)])
-def test_oracle_matches_reference_on_four_component_streams(oracle, built, tmp_path, w, h, sub, z):
-    from libjpeg_b200 import synth
-    data = oracle_binding.with_fourth_component(synth.encode(synth.source_image(w, h, 5), 80, sub, z, 1))
-    jpg = tmp_path / "f4.jpg"
-    jpg.write_bytes(data)
-    ref = oracle_binding.reference_decode(str(jpg), str(tmp_path / "f4.raw"))
-    assert ref is not None and ref.shape[2] == 4
-    rc, px = oracle.decode(data)
-    assert rc == 0 and np.array_equal(px, ref)
+@pytest.mark.parametrize("w,h,sub,z", FOUR_COMPONENT)
+def test_oracle_matches_reference_on_four_component_streams(oracle, built, w, h, sub, z):
+    ref = reference_decode("four", (w, h, sub, z))
+    assert ref is not None and ref["shape"][2] == 4
+    rc, px = oracle.decode(four_component_stream(w, h, sub, z))
+    assert rc == 0 and same_pixels(px, ref)
 
 
-@pytest.mark.skipif(not oracle_binding.have_reference(), reason="reference build (oracle/_ref) not present")
-@pytest.mark.parametrize("name", ["c420_96x80_z6_q75", "c444_64x64_z16_q90", "c422_100x60_z5_q80"])
-def test_oracle_without_color_transform_matches_reference_cli(oracle, tmp_path, name):
+@pytest.mark.parametrize("name", NO_COLOR_TRANSFORM)
+def test_oracle_without_color_transform_matches_reference_cli(oracle, name):
     """JPGTAG_MATRIX_LTRAFO = none (`jpeg -c` on decoding, cmd/main.cpp / reconstruct.cpp:336): Y, Cb, Cr upsampled, untransformed."""
-    import subprocess
-    src = os.path.join(GOLDEN, name + ".jpg")
-    ppm = tmp_path / "o.ppm"
-    r = subprocess.run([oracle_binding.REF_CLI, "-c", src, str(ppm)], capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr
-    raw = ppm.read_bytes()
-    magic, dims, maxv, rest = raw.split(b"\n", 3)
-    w, h = map(int, dims.split())
-    ref = np.frombuffer(rest, dtype=np.uint8).reshape(h, w, 3)
-    rc, px = oracle.decode_without_color_transform(open(src, "rb").read())
-    assert rc == 0 and np.array_equal(px, ref)
+    ref = reference_decode("nocolor", name)
+    rc, px = oracle.decode_without_color_transform(open(os.path.join(GOLDEN, name + ".jpg"), "rb").read())
+    assert rc == 0 and same_pixels(px, ref)
 
 
 def test_oracle_planes_match_reference_without_upsampling(oracle):
